@@ -3,7 +3,7 @@
 (CosineRandomFeatures 440 -> D = 16 x 4096 = 65536, BlockLeastSquaresEstimator(4096, numIter=1, lambda=1), k = 1000,
 N = 1M rows sharded over the GPUs of one node; strong scaling).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P bench.py --gpus N ...
 
 A "step" is one complete fit over the whole batch, ending with the fitted model (all W_j, feature means, intercept) in
@@ -66,7 +66,15 @@ def parse_args():
     ap.add_argument("--no-fast-mode", action="store_true")
     ap.add_argument("--precision", default=os.environ.get("KS_BENCH_PRECISION", "f16x2"), choices=["tf32", "f16", "f16x2"],
                     help="operand mode of the top-level numbers (fp32 accumulate, fp64 solve in every mode)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the model fitted by the last timed step of the top-level mode to DIR/*.npy "
+                         "(fp64; the weights as a fixed, seeded row sample, at most 64 MB in all), for comparing two builds")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
+    return args
 
 
 # ----------------------------------------------------------------------------------------- workload
@@ -94,6 +102,31 @@ def alg_flops(n, d_in, D, b, k, nb, num_iter=1):
     first = 2.0 * n * D * b + 4.0 * n * D * k + 2.0 * n * d_in * D + nb * (b ** 3 / 3.0 + 2.0 * b * b * k)
     more = (num_iter - 1) * (4.0 * n * D * k + 2.0 * n * d_in * D + nb * 2.0 * b * b * k)
     return first + more
+
+
+DUMP_BYTES = 64_000_000
+
+
+def dump_model(model, out_dir: str, seed: int = 0) -> dict:
+    """Writes what a caller of the fit receives: the feature means (D) and the intercept (k) whole, and the weights W (D x k,
+    524 MB at config 3) as the rows at a fixed, seeded, sorted sample of row indices, as many as fit the 64 MB budget.
+    Returns {file name: shape}."""
+    xs = model.xs
+    d, k = sum(w.shape[0] for w in xs), xs[0].shape[1]
+    means = np.concatenate(model.feature_means)
+    header = 4 * 128                                                    # one .npy header per file, the index file included
+    n_rows = min(d, (DUMP_BYTES - header - means.nbytes - 8 * k) // (8 * (k + 1)))
+    rows = np.sort(np.random.default_rng(seed).choice(d, size=n_rows, replace=False))
+    offs = np.cumsum([0] + [w.shape[0] for w in xs])
+    blk = np.searchsorted(offs, rows, side="right") - 1
+    arrays = {"W_sample": np.stack([xs[j][r - offs[j]] for j, r in zip(blk, rows)]),
+              "W_sample_rows": rows.astype(np.float64),
+              "feature_means": means,
+              "intercept": np.array(model.b_opt)}
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.ascontiguousarray(a, dtype=np.float64))
+    return {name: list(a.shape) for name, a in arrays.items()}
 
 
 # ----------------------------------------------------------------------------------------- clocks
@@ -286,7 +319,7 @@ def main():
     y_dev = ctx.labels_from_classes(cp.numpy(), args.classes)
     feats = feats_of(x_dev)
 
-    def resident_leg(precision, steps, warmup, sample_clocks):
+    def resident_leg(precision, steps, warmup, sample_clocks, keep_last=False):
         est = ks.BlockLeastSquaresEstimator(args.block, args.num_iter, args.lam, precision=precision)
         for _ in range(warmup):
             touch(est.fit(feats, y_dev))
@@ -295,19 +328,28 @@ def main():
         if sampler:
             sampler.start()
         l0 = ctx.launch_count()
-        stats, step_wall = [], []
+        stats, step_wall, last = [], [], None
         t0 = time.perf_counter()
-        for _ in range(steps):
+        for i in range(steps):
             ts = time.perf_counter()
-            touch(est.fit(feats, y_dev))
+            if keep_last and i == steps - 1:
+                last = est.fit(feats, y_dev)
+                touch(last)
+            else:
+                touch(est.fit(feats, y_dev))
             step_wall.append(1e3 * (time.perf_counter() - ts))
             stats.append(ctx.last_fit_stats())
         barrier()
         t = max_over_ranks((time.perf_counter() - t0) / steps)
         return {"t": t, "launches": (ctx.launch_count() - l0) // max(steps, 1), "clocks": sampler.stop() if sampler else None,
-                "dev_ms": max_over_ranks(float(np.mean([s["total_ms"] for s in stats]))), "step_wall": step_wall, "stats": stats[-1]}
+                "dev_ms": max_over_ranks(float(np.mean([s["total_ms"] for s in stats]))), "step_wall": step_wall, "stats": stats[-1],
+                "model": last}
 
-    main_leg = resident_leg(args.precision, args.steps, args.warmup, True)
+    main_leg = resident_leg(args.precision, args.steps, args.warmup, True, keep_last=args.dump_outputs is not None)
+    last_model, dumped = main_leg.pop("model"), None
+    if last_model is not None and rank == 0:                 # every rank holds the same model
+        dumped = dump_model(last_model, args.dump_outputs)
+    del last_model
     fast_leg = None
     if args.precision != "f16" and not args.no_fast_mode:
         fast_leg = resident_leg("f16", args.steps, args.warmup, False)
@@ -454,6 +496,8 @@ def main():
             out["fast_mode"]["e2e"] = e2e_fast
     if parity:
         out["parity"] = parity
+    if dumped:
+        out["dumped_outputs"] = {"dir": args.dump_outputs, "arrays": dumped}
     if cpu_baseline:
         out["cpu_baseline"] = cpu_baseline
     print(json.dumps(out))
